@@ -3,6 +3,7 @@
 1M x 256 fp32, 512-point C grid x 5 folds (BASELINE.json configs[1]).
 
     python bench.py [--gpus N] [--steps K] [--warmup W]            # this repo's CUDA path
+    python bench.py ... --dump-outputs DIR                         # also write the last timed step's outputs
     python bench.py --impl reference [--steps K] [--warmup W]      # the reference's CPU path
     python bench.py --config {3,4,5} ...                           # the other BASELINE.json configs (bench_configs.py)
 
@@ -46,7 +47,13 @@ def parse():
     p.add_argument("--folds", type=int, default=5)
     p.add_argument("--cpu-sample", type=int, default=40, help="fits timed for cpu_baseline / compared for parity (0 = skip)")
     p.add_argument("--kernel", type=int, default=0, help="0 auto, 1 SIMT fp32, 2 tcgen05")
+    p.add_argument("--dump-outputs", metavar="DIR", default=None,
+                   help="write what the last timed step computed as DIR/<name>.npy (see dump_outputs)")
     a = p.parse_args()
+    if a.steps < 1:
+        p.error("--steps must be at least 1")
+    if a.dump_outputs and (a.config != 2 or a.impl != "b200"):
+        p.error("--dump-outputs writes the outputs of the headline workload's CUDA path (--config 2 --impl b200)")
     if a.config == 2:
         a.n = a.n or 1_000_000
         a.d = a.d or 256
@@ -210,6 +217,32 @@ def fold_ids(y, n_folds):
     return fold
 
 
+DUMP_LIMIT = 63 * 10 ** 6      # array bytes; with the .npy headers the files stay under 64 MB
+
+
+def dump_outputs(out_dir, res, correct, count, n_cols, rank, world, order, cost):
+    """--dump-outputs: the arrays one timed step returns (logreg_fit_batch's coef / n_iter / status / loss /
+    n_evals, linear_score_batch's correct / count), one row per (candidate, fold) column in candidate-major
+    order (column = candidate * folds + fold) whatever the dealing over ranks, written by rank 0 as
+    float32 / float64 .npy files.  column.npy lists the columns written: all of them, or, when they would
+    exceed 64 MB, a fixed seeded sample, so that two builds run with the same arguments compare row for row."""
+    from skdist_b200 import parallel
+    local = {"coef": res["coef"], "n_iter": res["n_iter"], "status": res["status"], "loss": res["loss"],
+             "n_evals": res["n_evals"], "correct": correct, "count": count}
+    full = {k: parallel.all_gather_blocks(v, n_cols, rank, world, order, cost=cost) for k, v in local.items()}
+    if rank != 0:
+        return
+    full = {k: v if v.dtype in (np.float32, np.float64) else v.astype(np.float64) for k, v in full.items()}
+    row_bytes = 8 + sum(v[0].nbytes for v in full.values())
+    cols = np.arange(n_cols)
+    if row_bytes * n_cols > DUMP_LIMIT:
+        cols = np.sort(np.random.default_rng(0).choice(n_cols, DUMP_LIMIT // row_bytes, replace=False))
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "column.npy"), cols.astype(np.float64))
+    for k, v in full.items():
+        np.save(os.path.join(out_dir, k + ".npy"), v[cols])
+
+
 def workload_name(a):
     return "DistGridSearchCV(LogisticRegression) %d-point C grid x %d folds, synthetic G1 %dx%d fp32" % (
         a.candidates, a.folds, a.n, a.d)
@@ -338,6 +371,8 @@ def main():
         dist.all_reduce(tt, op=dist.ReduceOp.MAX)
     t_steps = float(tt.item())
     value = n_cols * a.steps / t_steps
+    if a.dump_outputs:
+        dump_outputs(a.dump_outputs, res, correct, count, n_cols, rank, world, deal_order, col_cost)
 
     # ---- end-to-end arm: public API on host arrays (H2D + fits + scoring + D2H), refit excluded
     gs_times = []

@@ -22,10 +22,12 @@ Pinning status (see DESIGN.md "Oracle"):
   ``tests/golden/search_logreg_digits10_{raw,scaled}.npz`` hold the scores of the reference's
   unmodified ``_fit_and_score`` plus its own run-to-run envelope; ``logreg_oracle.fit_multinomial_lbfgs``
   reproduces the stored fp32 coefficients bit for bit (``tests/test_oracle.py``).
-* Live pins that need /root/reference (skipped where it is absent): the multi-model search
+* Pins on what the reference's own code returns, recorded by ``tests/golden/make_golden.py
+  --reference-pins`` into ``tests/golden/reference_pins.{npz,json}``: the multi-model search
   against the reference's ``_raw_sampler`` / ``_fit_one_fold`` / ``_get_results``
-  (``tests/test_search_host.py``) and the feature eliminator against its ``_fit_and_score_one`` /
-  ``_drop_col`` (``tests/test_eliminate_host.py``).
+  (``tests/test_search_host.py``), the feature eliminator against its ``_fit_and_score_one`` /
+  ``_drop_col`` (``tests/test_eliminate_host.py``), and the constructor signatures and public
+  names of every Dist* class (``tests/test_boundary_host.py``).
 * The SGD (``sgd_oracle.py``), logistic (``logreg_oracle.py``) and ridge (``ridge_oracle.py``)
   restatements are bit-identical to the installed scikit-learn estimators (``tests/test_oracle.py``,
   ``tests/test_multiclass_host.py``); trees are checked against scikit-learn directly, which the

@@ -1,8 +1,8 @@
 """Import the UNMODIFIED reference (``/root/reference/skdist``) under sklearn 1.9.
 
-TEST INFRASTRUCTURE (see oracle/__init__.py).  Works only where /root/reference
-exists (the build container); used by tests/golden/make_golden.py to produce
-the committed fixtures and by tests that are skipped when it is absent.
+TEST INFRASTRUCTURE (see oracle/__init__.py).  Works only where a source tree of the
+reference exists; used by tests/golden/make_golden.py to produce the committed
+fixtures, which the tests compare against without the reference.
 
 The reference targets sklearn<0.23.2.  Three in-memory patches make its
 hot-path modules importable without touching any file (SURVEY.md section 8c):

@@ -1,11 +1,14 @@
 """Generate tests/golden/*.npz by running the UNMODIFIED reference per-task functions
-(/root/reference/skdist/distribute/search.py:_fit_and_score) under oracle/refshim.py.
+(skdist/distribute/search.py:_fit_and_score of sk-dist) under oracle/refshim.py.
 
-Run in the build container only (needs /root/reference):
+Needs a source tree of the reference (oracle/refshim.py, SKDIST_REFERENCE_ROOT):
     python tests/golden/make_golden.py
+    python tests/golden/make_golden.py --reference-pins
 The fixtures pin (i) the oracle restatement oracle/search_oracle.py against the reference
-and (ii) the CUDA path against both (tests/test_gpu_parity.py).  Inputs are regenerated
-from seeds by skdist_b200.datasets, so only outputs are stored.
+and (ii) the CUDA path against both (tests/test_gpu_parity.py); reference_pins.{npz,json} hold
+what the reference's own classes and helpers return on the inputs of the host tests that are pinned
+to it, so that those tests run without the reference.  Inputs are regenerated from seeds by
+skdist_b200.datasets, so only outputs are stored.
 """
 import os
 import sys
@@ -169,8 +172,100 @@ def run_multinomial_case(name, X, y, grid, cv, max_iter, ref_search):
     print(name, "noise_flips", noise_flips.ravel(), "\n  noise_coef", np.round(noise_coef.ravel(), 5))
 
 
+def reference_pins():
+    """What the tests that pin the drop-in against the reference's own code compare with: the outputs of
+    the UNMODIFIED reference functions and classes on the tests' inputs, stored as
+    reference_pins.npz (arrays) and reference_pins.json (signatures, parameter sets)."""
+    import copy
+    import json
+    import warnings
+    from itertools import product
+    from sklearn.linear_model import SGDClassifier
+    from sklearn.metrics import check_scoring
+    from sklearn.model_selection import StratifiedKFold
+    from sklearn.tree import DecisionTreeClassifier
+    from skdist_b200.datasets import make_multiclass
+    from skdist_b200.distribute.ensemble import MAX_RAND_SEED
+    from tests.test_boundary_host import CLASSES, _params
+    from tests.test_eliminate_host import ELIMINATOR_CASES, _data, feature_sets
+    from tests.test_forest_host import lattice
+    from tests.test_multiclass_host import NEGATIVES_CASES, negatives_input
+    warnings.simplefilter("ignore")
+    ref_search, ref_mc, ref_ens = refshim.load()
+    arrays, meta = {}, {}
+
+    # constructor signatures and public names of every Dist* class (tests/test_boundary_host.py)
+    meta["surface"] = {}
+    for module, names in CLASSES.items():
+        mod = refshim.load_module("skdist.distribute." + module)
+        meta["surface"][module] = {n: {"params": _params(getattr(mod, n)),
+                                       "public": sorted(a for a in dir(getattr(mod, n)) if not a.startswith("_"))}
+                                   for n in names}
+
+    # per-task function of the search: mean_test_score and best_params_ (tests/test_oracle.py)
+    X, y = make_g1_classification(1500, 8, seed=5)
+    cands = list(ParameterGrid({"C": [0.1, 10.0]}))
+    a = search_oracle.search_cv(LogisticRegression(), cands, X, y, cv=3, task_fn=reference_task(ref_search))
+    arrays["task_mean_test_score"] = a["cv_results_"]["mean_test_score"]
+    meta["task_best_params"] = a["best_params_"]
+
+    # the multi-model search's _raw_sampler / _fit_one_fold / _get_results (tests/test_search_host.py); the
+    # Spark branch's copy of each (fold, param_set) task is emulated with deepcopy (see the test)
+    X, y = make_g1_classification(400, 5, seed=6)
+    models = [("a", LogisticRegression(), {"C": [0.01, 0.1, 1.0, 10.0]}),
+              ("b", LogisticRegression(fit_intercept=False), {"C": [0.5, 5.0], "tol": [1e-4, 1e-3]})]
+    folds = list(StratifiedKFold(4).split(X, y))
+    param_sets = ref_search._raw_sampler(models, n=3, random_state=11)
+    scores = [ref_search._fit_one_fold((f, copy.deepcopy(ps)), models, X, y, None, {})
+              for f, ps in product(folds, param_sets)]
+    results = ref_search._get_results(scores)
+    meta["multi_model"] = {"param_set": list(results["param_set"]),
+                           "model_index": [int(i) for i in results["model_index"]]}
+    arrays["multi_model_score"] = results["score"].values.astype(np.float64)
+
+    # the feature eliminator's _fit_and_score_one per feature set (tests/test_eliminate_host.py)
+    ref_elim = refshim.load_module("skdist.distribute.eliminate")
+    X, y = _data()
+    for i, (step, n_cv, min_keep) in enumerate(ELIMINATOR_CASES):
+        base = LogisticRegression(C=0.3)
+        scorer = check_scoring(base, scoring=None)
+        arrays["eliminator_scores_%d" % i] = np.array(
+            [np.mean([ref_elim._fit_and_score_one(idx, base, X, y, scorer, tr, te, False, {})
+                      for tr, te in StratifiedKFold(n_cv).split(X, y)])
+             for idx in feature_sets(X, y, step, min_keep)])
+
+    # the forest's _build_trees (tests/test_forest_host.py)
+    X, y = lattice(1500, 8, 3)
+    for i, s in enumerate(np.random.RandomState(5).randint(MAX_RAND_SEED, size=3)):
+        tr = ref_ens._build_trees(DecisionTreeClassifier(max_features="sqrt"), (), {}, X,
+                                  y.astype(np.float64)[:, None], None, s, 3, bootstrap=True)
+        arrays["build_trees_threshold_%d" % i] = tr.tree_.threshold
+        arrays["build_trees_children_left_%d" % i] = tr.tree_.children_left.astype(np.int32)
+    X, y = lattice(300, 4, 6)
+    arrays["get_oof"] = ref_ens.get_oof(LogisticRegression(), X, y, n_splits=3)[1]
+
+    # one-vs-rest with sc=None, and the max_negatives down-sampling (tests/test_multiclass_host.py)
+    X, y = make_multiclass(500, 6, 4, seed=8)
+    r = ref_mc.DistOneVsRestClassifier(SGDClassifier(random_state=0)).fit(X, y)
+    arrays["ovr_sgd_coef"] = np.stack([e.coef_[0] for e in r.estimators_])
+    X, y = negatives_input()
+    for i, (mn, method, rs) in enumerate(NEGATIVES_CASES):
+        Xr, yr = ref_mc._negatives_mask(X, y, max_negatives=mn, random_state=rs, method=method)
+        arrays["negatives_rows_%d" % i] = np.sort(Xr[:, 0].astype(np.int32))
+        assert yr.sum() == y.sum()
+
+    np.savez_compressed(os.path.join(HERE, "reference_pins.npz"), **arrays)
+    with open(os.path.join(HERE, "reference_pins.json"), "w") as f:
+        json.dump(meta, f, indent=1, sort_keys=True)
+        f.write("\n")
+    print("reference_pins:", sorted(arrays))
+
+
 def main():
     ref_search, _, _ = refshim.load()
+    if "--reference-pins" in sys.argv:
+        reference_pins()
+        return
     if "--multinomial-only" in sys.argv:
         dg = load_digits()
         grid = {"C": [0.01, 0.1, 1.0, 10.0]}

@@ -42,3 +42,29 @@ def test_parity_block_against_the_cpu_leg(fake_engine):
     ci, f = tasks[4]
     bad["split%d_test_score" % f][ci] -= 3 / 1000
     assert bench.parity_block(bad, tasks, scores, fold, Cs, 3)["max_flips_per_fold"] == 3
+
+
+def test_dump_outputs_in_column_order_and_capped(tmp_path, monkeypatch):
+    """--dump-outputs: rows go back to column order whatever the dealing, every file is float32 / float64, and
+    above the size cap the same seeded sample of columns is written on every run."""
+    import bench
+    n_cols, d = 40, 5
+    order = np.random.default_rng(3).permutation(n_cols)       # the order the columns were fitted in
+    res = {"coef": (order[:, None] * 10.0 + np.arange(d + 1)).astype(np.float32), "n_iter": order.astype(np.int32),
+           "status": np.zeros(n_cols, np.int32), "loss": order * 0.5, "n_evals": order.astype(np.int32) + 1}
+    correct, count = order.astype(np.int64), np.full(n_cols, 7, np.int64)
+    bench.dump_outputs(str(tmp_path / "all"), res, correct, count, n_cols, 0, 1, order, None)
+    got = {p.stem: np.load(p) for p in (tmp_path / "all").iterdir()}
+    assert set(got) == {"column", "coef", "n_iter", "status", "loss", "n_evals", "correct", "count"}
+    assert all(v.dtype in (np.float32, np.float64) for v in got.values())
+    np.testing.assert_array_equal(got["column"], np.arange(n_cols))
+    np.testing.assert_array_equal(got["coef"][:, 0], np.arange(n_cols) * 10.0)
+    np.testing.assert_array_equal(got["n_evals"], np.arange(n_cols) + 1)
+    row_bytes = 8 + 4 * (d + 1) + 8 * 6
+    monkeypatch.setattr(bench, "DUMP_LIMIT", 10 * row_bytes)
+    for run in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / run), res, correct, count, n_cols, 0, 1, order, None)
+    cols = np.load(tmp_path / "a" / "column.npy")
+    assert len(cols) == 10 and np.array_equal(cols, np.load(tmp_path / "b" / "column.npy"))
+    assert sum(p.stat().st_size - 128 for p in (tmp_path / "a").iterdir()) <= 10 * row_bytes
+    np.testing.assert_array_equal(np.load(tmp_path / "a" / "correct.npy"), cols)

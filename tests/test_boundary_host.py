@@ -1,13 +1,13 @@
 """The Python drop-in boundary (SURVEY section 8b): constructor signatures (names, order, defaults) and the
-public method surface of every Dist* class against the reference's own classes, imported from /root/reference
-under oracle/refshim.py (skipped where the reference tree is absent, e.g. on the GPU box)."""
+public method surface of every Dist* class against the reference's own classes, as recorded from the
+unmodified reference in tests/golden/reference_pins.json (tests/golden/make_golden.py --reference-pins)."""
 import inspect
+import json
+import os
 
 import pytest
 
-from oracle import refshim
-
-pytestmark = pytest.mark.skipif(not refshim.available(), reason="reference tree not present")
+PINS = os.path.join(os.path.dirname(__file__), "golden", "reference_pins.json")
 
 CLASSES = {
     "search": ["DistGridSearchCV", "DistRandomizedSearchCV", "DistMultiModelSearch"],
@@ -36,17 +36,18 @@ def _params(cls):
 @pytest.mark.parametrize("module", sorted(CLASSES))
 def test_constructors_and_public_surface_match_the_reference(module):
     import importlib
-    ref = refshim.load_module("skdist.distribute." + module)
     ours = importlib.import_module("skdist.distribute." + module)
+    with open(PINS) as f:
+        surface = json.load(f)["surface"][module]
     for name in CLASSES[module]:
-        want, got = _params(getattr(ref, name)), _params(getattr(ours, name))
+        ref = surface[name]
+        want, got = [tuple(p) for p in ref["params"]], _params(getattr(ours, name))
         if name in KWARGS_AS:
             assert want[-1][1], "the reference constructor no longer ends in **kwargs"
             k, d = KWARGS_AS[name]
             want = want[:-1] + [(k, False, repr(d))]
         assert got == want, name
-        public = lambda c: {n for n in dir(c) if not n.startswith("_")}
-        missing = public(getattr(ref, name)) - public(getattr(ours, name)) - CONDITIONAL
+        missing = set(ref["public"]) - {n for n in dir(getattr(ours, name)) if not n.startswith("_")} - CONDITIONAL
         assert not missing, (name, sorted(missing))
 
 

@@ -1,11 +1,17 @@
 """DistFeatureEliminator host logic on the test-double engine, pinned against the UNMODIFIED
-reference class where /root/reference is present (joblib branch, ref eliminate.py:163-184)."""
+reference class (joblib branch, ref eliminate.py:163-184) through the scores it computed,
+stored in tests/golden/reference_pins.npz."""
+import os
+
 import numpy as np
 import pytest
 from sklearn.linear_model import LogisticRegression
 
 from skdist.distribute.eliminate import DistFeatureEliminator
 from skdist_b200.datasets import make_g1_classification
+
+# (step, cv, min_features_to_select) of the reference pin
+ELIMINATOR_CASES = ((2, 3, 7), (3, 4, 3))
 
 
 def _data():
@@ -15,32 +21,33 @@ def _data():
     return X, y
 
 
+def feature_sets(X, y, step, min_keep):
+    """The feature sets dropped in turn, built as eliminate.py:131-154 builds them."""
+    d = X.shape[1]
+    coefs = LogisticRegression(C=0.3).fit(X, y).coef_
+    ranks = np.ravel(np.argsort((coefs ** 2).sum(axis=0)))[: d - min_keep]
+    sets, k = [np.array([])], 0
+    while k < d - min_keep:
+        k += step
+        sets.append(ranks[:k])
+    return sets
+
+
 @pytest.mark.filterwarnings("ignore")
 def test_eliminator_matches_reference_task_function(fake_engine):
     """The reference class itself cannot run under scikit-learn 1.9 (`check_cv` is called with three
     positional arguments, eliminate.py:125), so the pin is on what every task executes: the
     UNMODIFIED `_fit_and_score_one` / `_drop_col` (eliminate.py:22-38) for each (feature set, fold),
     with the feature sets built as eliminate.py:131-154 builds them."""
-    from oracle import refshim
-    if not refshim.available():
-        pytest.skip("reference tree not present")
-    ref_elim = refshim.load_module("skdist.distribute.eliminate")
-    from sklearn.metrics import check_scoring
-    from sklearn.model_selection import StratifiedKFold
+    gold = np.load(os.path.join(os.path.dirname(__file__), "golden", "reference_pins.npz"))
     X, y = _data()
     d = X.shape[1]
-    for step, n_cv, min_keep in ((2, 3, d // 2), (3, 4, 3)):
+    for i, (step, n_cv, min_keep) in enumerate(ELIMINATOR_CASES):
         base = LogisticRegression(C=0.3)
         ours = DistFeatureEliminator(base, None, step=step, cv=n_cv, min_features_to_select=min_keep).fit(X, y)
-        coefs = LogisticRegression(C=0.3).fit(X, y).coef_
-        ranks = np.ravel(np.argsort((coefs ** 2).sum(axis=0)))[: d - min_keep]
-        sets, k = [np.array([])], 0
-        while k < d - min_keep:
-            k += step
-            sets.append(ranks[:k])
-        scorer = check_scoring(base, scoring=None)
-        ref_scores = [np.mean([ref_elim._fit_and_score_one(idx, base, X, y, scorer, tr, te, False, {})
-                               for tr, te in StratifiedKFold(n_cv).split(X, y)]) for idx in sets]
+        sets = feature_sets(X, y, step, min_keep)
+        ref_scores = gold["eliminator_scores_%d" % i]
+        assert len(ref_scores) == len(sets)
         np.testing.assert_allclose(ours.scores_, ref_scores, atol=1e-12)
         best = int(np.argmax(ref_scores))
         exp_keep = np.delete(range(d), sets[best].astype(int)) if len(sets[best]) else np.arange(d)

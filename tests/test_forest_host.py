@@ -1,13 +1,16 @@
 """Host side of the forest path (no GPU): the random numbers drawn per tree and the wrapping of
-node arrays into scikit-learn trees; plus the live pin that the reference's own `_build_trees`
-yields scikit-learn's trees (so sklearn's RandomForestClassifier is a valid oracle)."""
+node arrays into scikit-learn trees; plus the pin that the reference's own `_build_trees`
+yields scikit-learn's trees (so sklearn's RandomForestClassifier is a valid oracle), on the trees
+it built as stored in tests/golden/reference_pins.npz."""
+import os
+
 import numpy as np
 import pytest
 from sklearn.ensemble import RandomForestClassifier
-from sklearn.tree import DecisionTreeClassifier
 
-from oracle import refshim
 from skdist_b200.distribute.ensemble import MAX_RAND_SEED, _make_sklearn_tree, _tree_inputs
+
+PINS = os.path.join(os.path.dirname(__file__), "golden", "reference_pins.npz")
 
 
 def lattice(n, d, seed, levels=16):
@@ -43,17 +46,13 @@ def test_wrapping_roundtrip():
     np.testing.assert_array_equal(est.apply(X), rf.estimators_[0].apply(X))
 
 
-@pytest.mark.skipif(not refshim.available(), reason="reference tree not present")
 def test_reference_build_trees_equals_sklearn():
-    _, _, ref_ens = refshim.load()
+    gold = np.load(PINS)
     X, y = lattice(1500, 8, 3)
-    states = np.random.RandomState(5).randint(MAX_RAND_SEED, size=3)
     ref = RandomForestClassifier(n_estimators=3, random_state=5).fit(X, y)
-    for s, t in zip(states, ref.estimators_):
-        tr = ref_ens._build_trees(DecisionTreeClassifier(max_features="sqrt"), (), {}, X,
-                                  y.astype(np.float64)[:, None], None, s, 3, bootstrap=True)
-        np.testing.assert_array_equal(tr.tree_.threshold, t.tree_.threshold)
-        np.testing.assert_array_equal(tr.tree_.children_left, t.tree_.children_left)
+    for i, t in enumerate(ref.estimators_):
+        np.testing.assert_array_equal(gold["build_trees_threshold_%d" % i], t.tree_.threshold)
+        np.testing.assert_array_equal(gold["build_trees_children_left_%d" % i], t.tree_.children_left)
 
 
 def test_native_bootstrap_counts_equal_numpy():
@@ -247,7 +246,4 @@ def test_out_of_fold_helpers():
     assert oof.shape == (300, 2) and np.allclose(oof.sum(1), 1.0) and hasattr(clf, "coef_")
     idx, p = get_single_oof(LogisticRegression(), X, y, np.arange(100, 300), np.arange(100))
     np.testing.assert_allclose(p, oof[:100], rtol=1e-12)
-    if refshim.available():
-        ref = refshim.load_module("skdist.distribute.ensemble")
-        _, want = ref.get_oof(LogisticRegression(), X, y, n_splits=3)
-        np.testing.assert_array_equal(oof, want)
+    np.testing.assert_array_equal(oof, np.load(PINS)["get_oof"])

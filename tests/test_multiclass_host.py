@@ -1,6 +1,8 @@
 """DistOneVsRestClassifier host logic (no GPU) against scikit-learn's OneVsRestClassifier, which the
 reference's DistOneVsRestClassifier equals bit for bit when run unmodified with sc=None
-(SURVEY.md section 8c; live check in test_reference_ovr_equals_sklearn)."""
+(SURVEY.md section 8c; checked in test_reference_ovr_equals_sklearn on the coefficients the reference
+computed, stored in tests/golden/reference_pins.npz)."""
+import os
 import pickle
 import warnings
 
@@ -9,9 +11,22 @@ import pytest
 from sklearn.linear_model import LogisticRegression, SGDClassifier
 from sklearn.multiclass import OneVsRestClassifier
 
-from oracle import refshim, sgd_oracle
+from oracle import sgd_oracle
 from skdist.distribute.multiclass import DistOneVsRestClassifier
 from skdist_b200.datasets import make_multiclass
+
+PINS = os.path.join(os.path.dirname(__file__), "golden", "reference_pins.npz")
+# (max_negatives, method, random_state) of the reference's _negatives_mask pin
+NEGATIVES_CASES = [(mn, method, rs) for mn, method in [(300, "ratio"), (0.2, "ratio"), (2, "multiplier"),
+                                                       (1.5, "multiplier"), (10 ** 6, "ratio")] for rs in (0, 7)]
+
+
+def negatives_input():
+    rng = np.random.default_rng(0)
+    n = 5000
+    X = np.arange(n, dtype=np.float64)[:, None]
+    y = (rng.random(n) < 0.07).astype(int)
+    return X, y
 
 
 def test_ovr_logreg_matches_sklearn(fake_engine):
@@ -66,17 +81,16 @@ def test_ovr_sgd_matches_sklearn(fake_engine):
     np.testing.assert_array_equal(ovr.predict(X), ref.predict(X))
 
 
-@pytest.mark.skipif(not refshim.available(), reason="reference tree not present")
 @pytest.mark.filterwarnings("ignore")
 def test_reference_ovr_equals_sklearn():
-    """Live pin of the oracle choice: the UNMODIFIED reference DistOneVsRestClassifier (sc=None)
+    """Pin of the oracle choice: the UNMODIFIED reference DistOneVsRestClassifier (sc=None)
     equals sklearn's OneVsRestClassifier coefficient for coefficient."""
-    _, ref_multiclass, _ = refshim.load()
+    want = np.load(PINS)["ovr_sgd_coef"]
     X, y = make_multiclass(500, 6, 4, seed=8)
-    r = ref_multiclass.DistOneVsRestClassifier(SGDClassifier(random_state=0)).fit(X, y)
     s = OneVsRestClassifier(SGDClassifier(random_state=0)).fit(X, y)
-    for a, b in zip(r.estimators_, s.estimators_):
-        np.testing.assert_array_equal(a.coef_, b.coef_)
+    assert len(s.estimators_) == len(want)
+    for a, b in zip(want, s.estimators_):
+        np.testing.assert_array_equal(a, b.coef_[0])
 
 
 @pytest.mark.filterwarnings("ignore")
@@ -121,20 +135,13 @@ def test_negatives_rows_match_reference():
     """`max_negatives` down-sampling: the training rows of a label column equal the rows the
     reference's `_negatives_mask` (ref multiclass.py:76-106) keeps, for every method / type of
     `max_negatives` / random_state."""
-    if not refshim.available():
-        pytest.skip("reference tree not present")
     from skdist_b200.distribute.multiclass import _negatives_rows
-    _, mc, _ = refshim.load()
-    rng = np.random.default_rng(0)
-    n = 5000
-    X = np.arange(n, dtype=np.float64)[:, None]
-    y = (rng.random(n) < 0.07).astype(int)
-    for mn, method in [(300, "ratio"), (0.2, "ratio"), (2, "multiplier"), (1.5, "multiplier"), (10 ** 6, "ratio")]:
-        for rs in (0, 7):
-            Xr, yr = mc._negatives_mask(X, y, max_negatives=mn, random_state=rs, method=method)
-            rows = np.sort(Xr[:, 0].astype(int))
-            np.testing.assert_array_equal(rows, np.flatnonzero(_negatives_rows(y == 1, mn, rs, method)))
-            assert yr.sum() == y.sum()
+    gold = np.load(PINS)
+    _, y = negatives_input()
+    for i, (mn, method, rs) in enumerate(NEGATIVES_CASES):
+        rows = gold["negatives_rows_%d" % i]
+        np.testing.assert_array_equal(rows, np.flatnonzero(_negatives_rows(y == 1, mn, rs, method)))
+        assert y[rows].sum() == y.sum()
 
 
 def test_ovr_max_negatives_and_multilabel_host(fake_engine):

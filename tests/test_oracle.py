@@ -9,7 +9,7 @@ from sklearn.linear_model import LogisticRegression
 from sklearn.model_selection import ParameterGrid
 
 from oracle import logreg_oracle as lo
-from oracle import refshim, search_oracle
+from oracle import search_oracle
 from skdist_b200.datasets import make_g1_classification
 
 GOLD = os.path.join(os.path.dirname(__file__), "golden")
@@ -55,18 +55,17 @@ def test_logreg_restatement_is_bit_identical_to_sklearn():
             assert lo.accuracy(X, yf, coef, b) == m.score(X, y)
 
 
-@pytest.mark.skipif(not refshim.available(), reason="reference tree not present")
 @pytest.mark.filterwarnings("ignore")
 def test_oracle_task_equals_reference_task():
-    """Live pin: reference _fit_and_score (search.py:180-288) vs oracle.fit_and_score."""
-    from tests.golden.make_golden import reference_task
-    ref_search, _, _ = refshim.load()
+    """Pin: reference _fit_and_score (search.py:180-288), as stored in reference_pins.*, vs oracle.fit_and_score."""
+    import json
     X, y = make_g1_classification(1500, 8, seed=5)
     cands = list(ParameterGrid({"C": [0.1, 10.0]}))
-    a = search_oracle.search_cv(LogisticRegression(), cands, X, y, cv=3, task_fn=reference_task(ref_search))
     b = search_oracle.search_cv(LogisticRegression(), cands, X, y, cv=3)
-    np.testing.assert_array_equal(a["cv_results_"]["mean_test_score"], b["cv_results_"]["mean_test_score"])
-    assert a["best_params_"] == b["best_params_"]
+    np.testing.assert_array_equal(np.load(os.path.join(GOLD, "reference_pins.npz"))["task_mean_test_score"],
+                                  b["cv_results_"]["mean_test_score"])
+    with open(os.path.join(GOLD, "reference_pins.json")) as f:
+        assert json.load(f)["task_best_params"] == b["best_params_"]
 
 
 @pytest.mark.parametrize("dtype", [np.float32, np.float64])

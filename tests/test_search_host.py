@@ -122,35 +122,32 @@ def test_multi_model_search_matches_reference_semantics(fake_engine):
 
 @pytest.mark.filterwarnings("ignore")
 def test_multi_model_search_against_reference_functions(fake_engine):
-    """Live pin against the UNMODIFIED reference: its `_raw_sampler`, `_fit_one_fold` and
+    """Pin against the UNMODIFIED reference: its `_raw_sampler`, `_fit_one_fold` and
     `_get_results` (ref search.py:71-177) on the same inputs must give our cv_results_.  (The reference's own
     `DistMultiModelSearch.fit` raises NameError whenever random_state is set — `i` is undefined at
-    search.py:810 — so the pin is on the functions it calls.)  Skipped where /root/reference is absent."""
-    from oracle import refshim
-    if not refshim.available():
-        pytest.skip("reference tree not present")
+    search.py:810 — so the pin is on the functions it calls.)  What they returned is stored in
+    tests/golden/reference_pins.* (tests/golden/make_golden.py --reference-pins).
+
+    The Spark branch of `_fit_batch` (search.py:137-146) ships a pickled COPY of every
+    (fold, param_set) task to `_fit_one_fold`; its joblib branch passes the same dict object for
+    every fold, so each fold overwrites the previous fold's "score" (search.py:109-111) and the
+    "mean" becomes the last fold's score.  The Spark semantics are the intended ones: the stored
+    results emulate them."""
+    import json
+    import os
     from skdist_b200.distribute.search import DistMultiModelSearch
-    ref_search, _, _ = refshim.load()
-    from sklearn.model_selection import StratifiedKFold
+    gold = os.path.join(os.path.dirname(__file__), "golden", "reference_pins")
+    with open(gold + ".json") as f:
+        results = json.load(f)["multi_model"]
+    score = np.load(gold + ".npz")["multi_model_score"]
     X, y = make_g1_classification(400, 5, seed=6)
     models = [("a", LogisticRegression(), {"C": [0.01, 0.1, 1.0, 10.0]}),
               ("b", LogisticRegression(fit_intercept=False), {"C": [0.5, 5.0], "tol": [1e-4, 1e-3]})]
-    folds = list(StratifiedKFold(4).split(X, y))
-    param_sets = ref_search._raw_sampler(models, n=3, random_state=11)
-    # The Spark branch of `_fit_batch` (search.py:137-146) ships a pickled COPY of every
-    # (fold, param_set) task to `_fit_one_fold`; its joblib branch passes the same dict object for
-    # every fold, so each fold overwrites the previous fold's "score" (search.py:109-111) and the
-    # "mean" becomes the last fold's score.  The Spark semantics are the intended ones: emulate them.
-    import copy
-    from itertools import product
-    scores = [ref_search._fit_one_fold((f, copy.deepcopy(ps)), models, X, y, None, {})
-              for f, ps in product(folds, param_sets)]
-    results = ref_search._get_results(scores)
     ms = DistMultiModelSearch(models, None, n=3, cv=4, random_state=11).fit(X, y)
-    assert ms.cv_results_["params"] == list(results["param_set"])
-    assert ms.cv_results_["model_index"] == list(results["model_index"])
-    np.testing.assert_allclose(ms.cv_results_["mean_test_score"], results["score"].values, atol=1e-12)
-    assert ms.best_params_ == results.iloc[int(np.argmax(results["score"].values))]["param_set"]
+    assert ms.cv_results_["params"] == results["param_set"]
+    assert ms.cv_results_["model_index"] == results["model_index"]
+    np.testing.assert_allclose(ms.cv_results_["mean_test_score"], score, atol=1e-12)
+    assert ms.best_params_ == results["param_set"][int(np.argmax(score))]
 
 
 @pytest.mark.filterwarnings("ignore")
